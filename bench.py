@@ -17,6 +17,13 @@ voxel pooling (the two kernels BASELINE.json's metric names), all timed live wit
 `cpu_baseline` = the CPU oracle (port of the reference's PyTorch path) on the host cores, bounded sample, per segment.
 `--impl reference` times that CPU path alone (the reference itself is Python under mmcv and cannot travel to the GPU
 box; see DESIGN.md).
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as .npy files, so that two builds
+can be compared output for output (inputs and weights are seeded: the same arguments give the same inputs):
+  voxel_index.npy    (n,)    float64, flat indices into the (batch, X, Y, Z) output grid, sorted
+  output_voxels.npy  (n, K)  float32, class logits of ``output_voxels`` at those voxels
+  output_labels.npy  (n,)    float32, ``output_labels`` (argmax class) at those voxels
+n is every voxel when the three arrays fit in 48 MB, else a fixed seeded sample of that size.
 """
 import argparse
 import json
@@ -243,12 +250,13 @@ def cpu_threads():
 
 
 def cpu_measure(threads, max_timed, budget_s):
-    """1 warm-up + up to max_timed timed samples inside budget_s; returns (median seconds per sample, per-segment medians, k)."""
+    """1 warm-up + up to max_timed timed samples inside budget_s (exactly max_timed when budget_s is None); returns (median
+    seconds per sample, per-segment medians, k)."""
     step = cpu_sample(threads)
     t0 = time.perf_counter()
     _, seg0 = step()
     est = time.perf_counter() - t0
-    k = max(1, min(max_timed, int(budget_s / max(est, 1e-3))))
+    k = max_timed if budget_s is None else max(1, min(max_timed, int(budget_s / max(est, 1e-3))))
     segs = []
     for _ in range(k):
         _, sg = step()
@@ -261,10 +269,10 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     threads = cpu_threads()
-    per, seg, k, warm = cpu_measure(threads, args.steps, 170.0)
+    per, seg, k, warm = cpu_measure(threads, args.steps, None)
     val = 1.0 / per
     sample = (f"1 sample/step of {WORKLOAD} (connected: {', '.join(STAGES_ALL)}) through the CPU oracle port, fp32, "
-              f"{threads} threads of {os.cpu_count()} cores; 1 warm-up ({warm:.1f} s) + median of {k} timed steps (requested {args.steps})")
+              f"{threads} threads of {os.cpu_count()} cores; 1 warm-up ({warm:.1f} s) + median of {k} timed steps")
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": k,
             "warmup": 1, "ms_per_step": per * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
@@ -410,6 +418,27 @@ def rooflines(pipe, dev, peak):
     return conv, {"window_attn": wattn, "swin_qkv_attn_fused": fused_attn, "conv_c256": conv256, "voxel_pool": pool}
 
 
+DUMP_BYTES = 48 * 1000 * 1000
+
+
+def sample_outputs(voxels, labels):
+    """Host copies of one step's outputs for --dump-outputs (module docstring): voxels (B, K, X, Y, Z) float32 and
+    labels (B, X, Y, Z) at every voxel, or at a fixed seeded sample of voxels when that would exceed DUMP_BYTES."""
+    B, K = voxels.shape[:2]
+    nvox = labels.numel()
+    n = min(nvox, DUMP_BYTES // (8 + 4 * K + 4))
+    if n == nvox:
+        idx = torch.arange(nvox)
+    else:
+        idx = torch.randperm(nvox, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    d = idx.to(voxels.device)
+    per_b = nvox // B
+    vox = voxels.reshape(B, K, per_b)[d // per_b, :, d % per_b]  # (n, K)
+    return {"voxel_index": idx.double().numpy(),
+            "output_voxels": vox.float().cpu().numpy(),
+            "output_labels": labels.reshape(-1)[d].float().cpu().numpy()}
+
+
 def run_b200(args, rank, world, local_rank):
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
@@ -471,13 +500,15 @@ def run_b200(args, rank, world, local_rank):
         flush.fill_(float(i))  # L2 flush between timed iterations (untimed)
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        step_resident()
+        out = step_resident()
         b.record()
         evs.append((a, b))
     barrier()
     launches = (launches_per_step * args.steps) if graph is not None else ops.LAUNCH_COUNT[0] - launches0
     t_dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     clocks = sampler.stop() if rank == 0 else None
+    # copied now: the e2e steps below overwrite the graph's output buffers
+    dump = sample_outputs(out, pipe.labels) if args.dump_outputs and rank == 0 else None
 
     # ---------------------------------------------------------------- e2e: host buffers in, host result out
     # every step: H2D of the step's inputs from pinned host memory, the registered modules' forward, D2H of the per-voxel
@@ -554,6 +585,11 @@ def run_b200(args, rank, world, local_rank):
             "e2e": {"value": e2e_val, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                     "ms_per_step": t_e2e_ms / e2e_steps},
             "gpu_launches": launches, "roofline": roof, "roofline_extra": roof_extra, "cpu_baseline": cpu, "eval": eval_info}
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line), flush=True)
 
 
@@ -571,7 +607,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch eagerly instead of replaying a captured CUDA graph")
     ap.add_argument("--precision", default="fp32", choices=["fp32", "bf16"],
                     help="fp32 (default, graded): three bf16 passes on split operands; bf16: single pass (config 5's mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     set_workload(args.workload)
     rank = int(os.environ.get("RANK", "0"))
